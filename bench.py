@@ -1,5 +1,5 @@
 #!/usr/bin/env python
-"""bench.py — headline benchmark of the DASR SRN hot path on B200 (contract in the task statement).
+"""bench.py — headline benchmark of the DASR SRN hot path on B200; prints one JSON result line on stdout.
 
 Workload (BASELINE.json configs[1]): RRDBNet-23 x4 generator forward, batch 16 x 3 x 256 x 256 synthetic LR
 images per GPU (weak scaling), tcgen05 bf16 kernels (fp32 accumulate), random-init weights of the
@@ -12,8 +12,13 @@ reference architecture.  metric = output megapixels / second over all GPUs.
   cpu_baseline  : the oracle port of the reference forward on the host cores (bounded sample)
   train         : DASR_Model train step (BASELINE configs[2]: B=32, HR crop 128) iterations / second, fp32 kernels
 
-`--impl reference` times the reference algorithm's CPU path (oracle port: the reference is pure Python and
-/root/reference does not exist on the GPU box) on the host cores with all threads.
+`--impl reference` times the reference algorithm's CPU path (oracle port of the pure-Python reference) on the host
+cores with all threads.
+
+`--steps K` is the number of timed steps of every GPU forward measurement and of `--impl reference`; the cpu_baseline
+sample beside the GPU result is one forward (it only sets the scale of the comparison).  `--dump-outputs DIR` writes what
+the timed GPU forward returned in its last step (see dump_outputs), so that two builds can be compared output for
+output: inputs and weights are generated from fixed seeds and are identical from run to run.
 """
 import argparse
 import json
@@ -179,11 +184,28 @@ def cpu_reference_dsn_step(threads, B=4):
     return (B / 8.0) / dt, dt
 
 
+DUMP_SAMPLES = 1 << 22
+
+
+def dump_outputs(dirname, sr):
+    """Write the SR batch of one forward ([16, 3, 1024, 1024], 201 MB as float32) as a fixed, seeded sample of
+    DUMP_SAMPLES elements: DIR/sr.npy holds their values (float32), DIR/sr_index.npy their flat positions in the batch
+    (ascending, float64: exact).  48 MB in all."""
+    import numpy as np
+    import torch
+    os.makedirs(dirname, exist_ok=True)
+    flat = sr.detach().float().reshape(-1)
+    idx = np.sort(np.random.default_rng(0).choice(flat.numel(), size=DUMP_SAMPLES, replace=False))
+    vals = flat[torch.from_numpy(idx).to(flat.device)].cpu().numpy()
+    np.save(os.path.join(dirname, 'sr.npy'), vals)
+    np.save(os.path.join(dirname, 'sr_index.npy'), idx.astype(np.float64))
+
+
 def run_reference(args, rank):
     if rank != 0:
         return
     threads = pick_threads()
-    steps, warm = max(1, min(args.steps, 2)), 1 if args.warmup > 0 else 0
+    steps, warm = args.steps, 1 if args.warmup > 0 else 0
     nimg = 4
     mp_s, dt = cpu_reference_forward(nimg, LR, threads, steps, warm)
     line = {
@@ -209,7 +231,12 @@ def main():
     ap.add_argument('--impl', default='dasr_b200')
     ap.add_argument('--train-steps', type=int, default=20)
     ap.add_argument('--no-cpu-baseline', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the output of the last timed forward step to DIR/*.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs writes the output of the GPU path; it does not apply to --impl reference')
     rank = int(os.environ.get('RANK', 0))
     local_rank = int(os.environ.get('LOCAL_RANK', 0))
     world = int(os.environ.get('WORLD_SIZE', 1))
@@ -228,7 +255,7 @@ def main():
     from dasr_b200 import _lib
     from dasr_b200.srn.models import create_model
     from dasr_b200.srn.options.options import dict_to_nonedict
-    W, K = max(args.warmup, 3), max(args.steps, 1)
+    W, K = max(args.warmup, 3), args.steps
 
     def barrier():
         if world > 1:
@@ -279,6 +306,8 @@ def main():
         launches = _lib.LAUNCHES - l0
         ms = max_over_ranks(e0.elapsed_time(e1) / K)
         clocks = sampler.stop() if sampler else None
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, out)
         del out
         # roofline: time of the conv_tc launch sequence = step time minus the (few) non-conv kernels of a forward,
         # which are timed here on the same shapes: layout change of the input, zero fill, per-chunk feature copy,
@@ -355,11 +384,11 @@ def main():
                 netG(x_dev)
             barrier()
             e0.record()
-            for _ in range(min(K, 10)):
+            for _ in range(K):
                 out = netG(x_dev)
             e1.record()
             barrier()
-            fp16_ms = max_over_ranks(e0.elapsed_time(e1) / min(K, 10))
+            fp16_ms = max_over_ranks(e0.elapsed_time(e1) / K)
             del out
             netG.precision = 'bf16'
     model.fake_H = None

@@ -195,6 +195,9 @@ def gen_dasr_step(fs, name, ragan=False):
             G_delta_norm=float(sum(((G[k] - sdG[k]).double() ** 2).sum() for k in G) ** 0.5),
             D_delta_norm=float(sum(((D[k] - sdD[k]).double() ** 2).sum() for k in D) ** 0.5)))
         print('  step', step, {k: round(v, 6) for k, v in log.items()})
+    # one file per step keeps every fixture under 1 MB (tests/helpers.py load_train_steps)
+    for k, s in enumerate(rec.pop('steps'), 1):
+        save(name.replace('.pt', '.step%d.pt' % k), s)
     save(name, rec)
 
 

@@ -1,5 +1,5 @@
 """Generate tests/golden/f1_*.pt (SURVEY §8f.1: SRResNet + pixelshuffle, the BatchNorm VGG-style discriminators, the
-ESRGAN / SRGAN train steps) by running the UNMODIFIED reference on CPU.  Test infrastructure only.
+ESRGAN / SRGAN train steps; one file per case, each under 1 MB) by running the UNMODIFIED reference on CPU.  Test infrastructure only.
 
     python oracle/gen_golden_f1.py
 
@@ -95,7 +95,8 @@ def gen_modules():
     d = arch.Discriminator_VGG_192(3, 64, norm_type='batch', act_type='leakyrelu', mode='CNA')
     rec['vgg192'] = dict(w_seed=331, x_seed=332, x_shape=(2, 3, 192, 192), pat_seed=333,
                          **module_case(d, O.synth_image((2, 3, 192, 192), 332), 331, 333))
-    save('f1_modules.pt', rec)
+    for case, obj in rec.items():
+        save('f1_%s.pt' % case, obj)
 
 
 def make_opt(model):
@@ -135,7 +136,8 @@ def gen_steps():
                               D_running=OrderedDict((k, v.clone()) for k, v in D.items() if 'running' in k or 'num_batches' in k)))
             print(' ', model_name, 'step', step, {k: round(v, 6) for k, v in log.items()})
         rec[model_name] = dict(wG_seed=341, wD_seed=342, wF_seed=343, data_seeds=(351, 361), steps=steps)
-    save('f1_steps.pt', rec)
+    for model_name, obj in rec.items():
+        save('f1_steps_%s.pt' % model_name, obj)
 
 
 if __name__ == '__main__':

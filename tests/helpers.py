@@ -1,5 +1,14 @@
-"""Shared helpers of the GPU tests (importable as `helpers`: tests/conftest.py puts this directory on sys.path)."""
+"""Shared helpers of the tests (importable as `helpers`: tests/conftest.py puts this directory on sys.path)."""
 import torch
+
+
+def load_train_steps(golden, name):
+    """A train-step fixture `<stem>.pt` holds the configuration; each optimisation step is stored in `<stem>.step<k>.pt`
+    (k = 1, 2, ...), which keeps every file under 1 MB.  Returns the configuration with the list of steps under 'steps'."""
+    g = golden(name)
+    stem = name[:-len('.pt')]
+    g['steps'] = [golden('%s.step%d.pt' % (stem, k)) for k in range(1, len(g['data_seeds']) + 1)]
+    return g
 
 
 def make_opt(is_train, model, nb=1, fs='wavelet', gpu=True):

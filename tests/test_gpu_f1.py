@@ -70,24 +70,24 @@ def check_module(net, g):
 
 def test_srresnet_pixelshuffle_vs_reference(golden):
     from dasr_b200.srn.models.modules.architecture import SRResNet
-    g = golden('f1_modules.pt')['srresnet']
+    g = golden('f1_srresnet.pt')
     check_module(SRResNet(3, 3, 64, 2, upscale=4, norm_type=None, act_type='relu', mode='CNA', upsample_mode='pixelshuffle'), g)
 
 
 def test_srresnet_batchnorm_nac_upconv_vs_reference(golden):
     from dasr_b200.srn.models.modules.architecture import SRResNet
-    g = golden('f1_modules.pt')['srresnet_bn_nac']
+    g = golden('f1_srresnet_bn_nac.pt')
     check_module(SRResNet(3, 3, 32, 1, upscale=2, norm_type='batch', act_type='relu', mode='NAC', res_scale=0.5, upsample_mode='upconv'), g)
 
 
 def test_discriminator_vgg_128_vs_reference(golden):
     from dasr_b200.srn.models.modules.architecture import Discriminator_VGG_128
-    check_module(Discriminator_VGG_128(3, 64), golden('f1_modules.pt')['vgg128'])
+    check_module(Discriminator_VGG_128(3, 64), golden('f1_vgg128.pt'))
 
 
 def test_discriminator_vgg_192_vs_reference(golden):
     from dasr_b200.srn.models.modules.architecture import Discriminator_VGG_192
-    check_module(Discriminator_VGG_192(3, 64, norm_type='batch', act_type='leakyrelu', mode='CNA'), golden('f1_modules.pt')['vgg192'])
+    check_module(Discriminator_VGG_192(3, 64, norm_type='batch', act_type='leakyrelu', mode='CNA'), golden('f1_vgg192.pt'))
 
 
 @pytest.mark.parametrize('name', ['srragan', 'srgan'])
@@ -97,7 +97,7 @@ def test_srgan_train_steps_vs_reference(golden, name):
     from dasr_b200.srn.models import create_model
     from dasr_b200.srn.options.options import dict_to_nonedict
     from helpers import unwrap
-    g = golden('f1_steps.pt')[name]
+    g = golden('f1_steps_%s.pt' % name)
     opt = dict_to_nonedict({
         'name': 'golden', 'model': name, 'scale': 4, 'gpu_ids': [0], 'is_train': True, 'chop': False, 'val_lpips': False,
         'path': {'pretrain_model_G': None, 'pretrain_model_D': None, 'models': '/tmp', 'training_state': '/tmp'},

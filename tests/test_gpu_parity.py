@@ -381,7 +381,8 @@ def test_dasr_model_train_steps_vs_golden(golden, name):
     """create_model -> feed_data -> optimize_parameters x2 through the public API, against the log values
     and post-step weights the reference produced for the same inputs (oracle/gen_golden.py)."""
     from dasr_b200.srn.models import create_model
-    g = golden(name)
+    from helpers import load_train_steps
+    g = load_train_steps(golden, name)
     fs = g['fs']
     opt = make_opt(True, 'DASR', g['nb'], fs)
     opt['train']['ragan'] = bool(g.get('ragan', False))        # dasr_step_ragan.pt: relativistic average GAN terms

@@ -137,8 +137,8 @@ def test_mixed_precision_dasr_steps_vs_reference_fixture(golden, monkeypatch):
     compared through the UPDATE direction (cosine > 0.8: signs of near-zero gradients flip under bf16)."""
     monkeypatch.setenv('DASR_B200_TRAIN_PRECISION', 'bf16')
     from dasr_b200.srn.models import create_model
-    from helpers import make_opt, unwrap
-    g = golden('dasr_step_wavelet.pt')
+    from helpers import load_train_steps, make_opt, unwrap
+    g = load_train_steps(golden, 'dasr_step_wavelet.pt')
     model = create_model(make_opt(True, 'DASR', g['nb'], g['fs']))
     sdG = O.synth_state_dict(O.rrdbnet_shapes(nb=g['nb']), g['wG_seed'], g['gain_G'])
     sdD = O.synth_state_dict(O.nlayer_d_shapes(9, 64, 2), g['wD_seed'], 1.0)

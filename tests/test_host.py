@@ -2,6 +2,7 @@
 and the data-parallel gradient bucket over gloo with world_size 2."""
 import json
 import os
+import shlex
 import subprocess
 import sys
 
@@ -209,25 +210,62 @@ def test_dsn_modules_match_reference_state_dict_layout():
         net(torch.zeros(1, 3, 16, 16))
 
 
+def _write_tree(base, files):
+    for rel, text in files.items():
+        p = base / rel
+        p.parent.mkdir(parents=True, exist_ok=True)
+        p.write_text(text)
+
+
+# A stand-in for a DASR `codes` checkout: the directory layout and the top-level module names its entry scripts import.
+# Every module the dasr_b200 mirrors replace fails on import here, so a script that gets the checkout's own copy stops.
+def _decoy(name):
+    return 'raise ImportError("the checkout\'s own %s was imported instead of the dasr_b200 mirror")\n' % name
+
+
+SRN_DECOYS = {name: _decoy(name) for name in ('models/__init__.py', 'options/__init__.py', 'options/options.py',
+                                              'utils/__init__.py', 'utils/util.py')}
+DSN_DECOYS = {name: _decoy(name) for name in ('model.py', 'loss.py')}
+
+# SRN inference entry point: option file -> logger -> dataset -> create_model -> feed_data / test, like codes/SRN/test.py.
+SRN_TEST_SCRIPT = r'''
+import argparse
+import logging
+
+import options.options as option
+import utils.util as util
+from data import create_dataset
+from models import create_model
+from utils.receptive_cal import WINDOW      # a module only the checkout has: found through the mirror package's search path
+
+ap = argparse.ArgumentParser()
+ap.add_argument('-opt', required=True)
+opt = option.dict_to_nonedict(option.parse(ap.parse_args().opt, is_train=False))
+util.mkdirs([opt['path']['results_root'], opt['path']['log']])
+util.setup_logger(None, opt['path']['log'], 'test.log', level=logging.INFO, screen=True)
+model = create_model(opt)
+for batch in create_dataset(opt['datasets']['test_1']):
+    model.feed_data(batch, False)
+    model.test()
+'''
+SRN_DATA_PACKAGE = r'''
+import torch
+
+
+def create_dataset(opt):
+    return [{'LR': torch.rand(1, 3, 16, 16), 'LR_path': ['a.png']}]
+'''
+
+
 def test_reference_test_py_runs_unchanged_through_the_launcher(tmp_path):
-    """Drop-in boundary: the reference's own codes/SRN/test.py, executed unchanged by dasr_b200.launch, parses its JSON,
-    builds its dataset/dataloader with the reference's data/ package, creates the model through the mirror and reaches
-    the first kernel call — which must refuse loudly on this GPU-less host (no CPU fallback).  Skipped where the
-    reference checkout is absent (the GPU box)."""
+    """Drop-in boundary: an SRN test script, executed unchanged by dasr_b200.launch from a checkout whose own `models`,
+    `options` and `utils` packages sit next to it, parses its JSON, builds its dataset with the checkout's data/ package,
+    creates the model through the mirror and reaches the first kernel call — which must refuse loudly on a host without
+    a GPU (no CPU fallback)."""
     import json
-    import subprocess
-    import sys
-    import numpy as np
-    import pytest
-    ref = '/root/reference/codes/SRN/test.py'
-    if not os.path.exists(ref):
-        pytest.skip('reference checkout not present')
-    cv2 = pytest.importorskip('cv2')
-    rng = np.random.RandomState(0)
-    (tmp_path / 'LR').mkdir()
-    (tmp_path / 'HR').mkdir()
-    cv2.imwrite(str(tmp_path / 'LR' / 'a.png'), (rng.rand(16, 16, 3) * 255).astype(np.uint8))
-    cv2.imwrite(str(tmp_path / 'HR' / 'a.png'), (rng.rand(64, 64, 3) * 255).astype(np.uint8))
+    srn = tmp_path / 'codes' / 'SRN'
+    _write_tree(srn, dict(SRN_DECOYS, **{'test.py': SRN_TEST_SCRIPT, 'data/__init__.py': SRN_DATA_PACKAGE,
+                                          'utils/receptive_cal.py': 'WINDOW = 1\n'}))
     opt = {'name': 'dropin_test', 'suffix': None, 'model': 'sr', 'scale': 4, 'gpu_ids': None, 'chop': False, 'val_lpips': False,
            'save_RealorFake': False,
            'datasets': {'test_1': {'name': 'toy', 'mode': 'LRHR', 'dataroot_HR': str(tmp_path / 'HR'), 'dataroot_LR': str(tmp_path / 'LR')}},
@@ -236,38 +274,41 @@ def test_reference_test_py_runs_unchanged_through_the_launcher(tmp_path):
                          'gc': 32, 'group': 1}}
     cfg = tmp_path / 'test.json'
     cfg.write_text(json.dumps(opt))
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    env = dict(os.environ, PYTHONPATH=os.pathsep.join([root, os.path.join(root, 'oracle', 'ref_stubs')]), CUDA_VISIBLE_DEVICES='')
-    r = subprocess.run([sys.executable, '-m', 'dasr_b200.launch', ref, '-opt', str(cfg)], cwd=str(tmp_path), env=env,
+    env = dict(os.environ, PYTHONPATH=ROOT, CUDA_VISIBLE_DEVICES='')
+    r = subprocess.run([sys.executable, '-m', 'dasr_b200.launch', str(srn / 'test.py'), '-opt', str(cfg)], cwd=str(tmp_path), env=env,
                        capture_output=True, text=True, timeout=600)
     err = r.stderr + r.stdout
     assert r.returncode != 0
-    assert 'dasr_b200/srn/models/SR_model.py' in err, err[-2000:]          # the mirror, not the reference's models package
+    assert 'was imported instead of the dasr_b200 mirror' not in err, err[-2000:]
+    assert 'dasr_b200/srn/models/SR_model.py' in err, err[-2000:]          # the mirror, not the checkout's models package
     assert 'no CPU fallback exists' in err, err[-2000:]
 
 
 def test_auto_reproduce_resolves_to_the_mirrors_after_install(tmp_path):
-    """`python -m dasr_b200.install <codes>` + the unmodified Auto_Reproduce.py (Auto_Reproduce.py:38-40 shells out to
-    `cd ./DSN; sh auto_reproduce_launcher_<dataset>.sh` and `cd ./SRN; python train.py -opt ...`): both child scripts must
-    import the dasr_b200 mirrors although their own directory is first on sys.path.  The stages stop at the datasets
-    (no data here); the overlay log records which imports were redirected for which script directory."""
-    import shutil
-    import pytest
-    ref = '/root/reference/codes'
-    if not os.path.exists(os.path.join(ref, 'Auto_Reproduce.py')):
-        pytest.skip('reference checkout not present')
+    """`python -m dasr_b200.install <codes>` + an unmodified driver script that shells out like codes/Auto_Reproduce.py
+    (`cd ./DSN; sh <launcher>.sh` and `cd ./SRN; python train.py -opt ...`): both child scripts must import the dasr_b200
+    mirrors although their own directory is first on sys.path.  The overlay log records which imports were redirected for
+    which script directory."""
     codes = tmp_path / 'codes'
-    shutil.copytree(ref, str(codes), ignore=shutil.ignore_patterns('*.tar', '*.png', '*.jpg', '*.pyc', '__pycache__', '*.gif'))
+    py = shlex.quote(sys.executable)
+    _write_tree(codes, {
+        'Auto_Reproduce.py': 'import os\nos.system("cd ./DSN; sh launcher.sh")\nos.system("cd ./SRN; %s train.py -opt x.json")\n' % py,
+        'DSN/launcher.sh': '%s train.py --generator DeResnet\n' % py,
+        'DSN/train.py': 'import model\nimport loss\nimport utils\n',
+        'DSN/utils.py': '',
+        'SRN/train.py': 'import options.options\nimport utils.util\nimport models\n'})
+    _write_tree(codes / 'DSN', DSN_DECOYS)
+    _write_tree(codes / 'SRN', SRN_DECOYS)
     from dasr_b200 import install
     import io
     buf = io.StringIO()
     site_dir = install.install(str(codes), pth=False, out=buf)
     assert 'PYTHONPATH' in buf.getvalue() and (codes / 'SRN' / '.dasr_b200').read_text().strip() == 'SRN'
     log = tmp_path / 'overlay.log'
-    env = dict(os.environ, PYTHONPATH=os.pathsep.join([site_dir, ROOT, os.path.join(ROOT, 'oracle', 'ref_stubs')]),
+    env = dict(os.environ, PYTHONPATH=os.pathsep.join([site_dir, ROOT]),
                CUDA_VISIBLE_DEVICES='', DASR_B200_OVERLAY_LOG=str(log), DASR_B200_ALLOW_RANDOM_VGG='1')
-    r = subprocess.run([sys.executable, 'Auto_Reproduce.py', '--dataset', 'realsr', '--artifact', 'tdrealsr'], cwd=str(codes), env=env,
-                       capture_output=True, text=True, timeout=900)
+    r = subprocess.run([sys.executable, 'Auto_Reproduce.py'], cwd=str(codes), env=env, capture_output=True, text=True, timeout=900)
+    assert 'was imported instead of the dasr_b200 mirror' not in r.stdout + r.stderr, r.stderr[-3000:]
     text = log.read_text() if log.exists() else ''
     dsn_dir, srn_dir = str(codes / 'DSN'), str(codes / 'SRN')
     for name in ('model', 'loss'):

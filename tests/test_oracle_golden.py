@@ -73,7 +73,8 @@ def test_filters_losses_utils(golden):
 
 
 def _check_step(golden, name):
-    g = golden(name)
+    from helpers import load_train_steps
+    g = load_train_steps(golden, name)
     fs = g['fs']
     sdG = O.synth_state_dict(O.rrdbnet_shapes(nb=g['nb']), g['wG_seed'], g['gain_G'])
     sdD = O.synth_state_dict(O.nlayer_d_shapes(9 if fs == 'wavelet' else 3, 64, 2), g['wD_seed'], 1.0)

@@ -16,10 +16,9 @@ from dasr_b200.srn.models.modules.architecture import Discriminator_VGG_128, Dis
 
 torch.backends.cudnn.allow_tf32 = False
 torch.backends.cuda.matmul.allow_tf32 = False
-g = torch.load(os.path.join(ROOT, 'tests', 'golden', 'f1_modules.pt'))
 for name, net in (('vgg128', Discriminator_VGG_128(3, 64)),
                   ('vgg192', Discriminator_VGG_192(3, 64, norm_type='batch', act_type='leakyrelu', mode='CNA'))):
-    gg = g[name]
+    gg = torch.load(os.path.join(ROOT, 'tests', 'golden', 'f1_%s.pt' % name))
     net.load_state_dict(synth_sd(net, gg['w_seed']), strict=False)
     net.train()
     x = O.synth_image(gg['x_shape'], gg['x_seed'])
